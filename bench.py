@@ -13,6 +13,8 @@ semantics, every output bit-exact with the oracle -- tests/test_gpu_parity.py).
   cpu_baseline : the reference's algorithm (oracle/egs_oracle.c, a port) on this box's host cores
 
 `--impl reference` times that CPU port alone on the same workload (bounded sample per step).
+`--dump-outputs DIR` saves the per-pod outputs of the last timed step; the inputs are seeded, so two builds run with the
+same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -45,7 +47,14 @@ def parse():
     ap.add_argument("--no-roofline", action="store_true")
     ap.add_argument("--roofline-only", action="store_true", help="PROFILING ONLY: just the 4M-node k_evaluate leg (for ncu)")
     ap.add_argument("--no-configs", action="store_true", help="skip the side measurements of BASELINE configs 1-3")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the per-pod outputs of the last timed step as DIR/<field>.npy (see write_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and (args.impl != "b200" or args.roofline_only):
+        ap.error("--dump-outputs needs the timed steps of --impl b200")
+    return args
 
 
 def ncu_traffic():
@@ -195,6 +204,22 @@ def out_hash(out) -> str:
     for f in FIELDS:
         h.update(np.ascontiguousarray(out[f]).tobytes())
     return h.hexdigest()
+
+
+def write_outputs(dirname, out):
+    """The six per-pod output arrays of a batch as DIR/<field>.npy, in float dtypes that hold every value exactly:
+    node, status, fit_count [P] and alloc_mask [P, 4] as float32 (node ids and counts stay below 2^24); each 64-bit
+    digest as float64 [P, 2] = (low 32 bits, high 32 bits).  60 bytes per pod: 60 MB for the 1M-pod batch."""
+    os.makedirs(dirname, exist_ok=True)
+    for f in FIELDS:
+        a = np.asarray(out[f])
+        if f.endswith("_digest"):
+            u = a.astype(np.uint64)
+            a = np.stack([u & np.uint64(0xFFFFFFFF), u >> np.uint64(32)], axis=1).astype(np.float64)
+        else:
+            assert np.abs(a.astype(np.int64)).max(initial=0) < (1 << 24), f"{f} is not exact in float32"
+            a = a.astype(np.float32)
+        np.save(os.path.join(dirname, f + ".npy"), a)
 
 
 def sharded_handle(eg, w, rank, world, local, dist, sub=None):
@@ -359,6 +384,9 @@ def main():
     e.profile_reset(False)
     clocks.mark()
     ms_total = timed(step_resident, args.steps)
+    # the last timed step's outputs, copied before the untimed breakdown step below reuses the same buffers
+    last_out = ({f: t.cpu().numpy() for f, t in zip(FIELDS, (o_node, o_status, o_alloc, o_fit, o_fd, o_sd))}
+                if args.dump_outputs and rank == 0 else None)
     launches = sum(e.profile_get(k)[0] for k in range(8))
     ev_launches, ev_ms = e.profile_get(cap.EGS_K_EVALUATE)       # cold-shape table fills inside the timed steps
     clk = clocks.stop() if rank == 0 else None
@@ -502,6 +530,8 @@ def main():
     }
     if args.pods:
         line["profiling_subset"] = True
+    if last_out is not None:
+        write_outputs(args.dump_outputs, last_out)
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

@@ -103,7 +103,9 @@ def build_shim_double(force: bool = False) -> str:
     build_libegs(force)
     if force or _stale(SHIM_DOUBLE, [src, LIBEGS, os.path.join(ROOT, "include", "egs.h")]):
         os.makedirs(os.path.dirname(SHIM_DOUBLE), exist_ok=True)
-        subprocess.check_call(["gcc", "-O2", "-o", SHIM_DOUBLE, src, "-L" + LIBDIR, "-legs", "-Wl,-rpath," + LIBDIR])
+        # rpath relative to the binary, so a built tree still runs after it is copied or moved
+        rpath = os.path.join("$ORIGIN", os.path.relpath(LIBDIR, os.path.dirname(SHIM_DOUBLE)))
+        subprocess.check_call(["gcc", "-O2", "-o", SHIM_DOUBLE, src, "-L" + LIBDIR, "-legs", "-Wl,-rpath," + rpath])
     return SHIM_DOUBLE
 
 
