@@ -549,6 +549,25 @@ int egso_cache_load(egso *o, int C, const egso_unit *units, int n, const int32_t
   }
   return ST_OK;
 }
+/* TEST SUPPORT: the inverse of egso_cache_load, egso_peek over nodes [0, n) in one call: valid[i] = 1 when node i
+ * holds an entry of the shape, then score[i] and alloc_mask[i][c] as egso_cache_load takes them (0 otherwise). */
+int egso_cache_dump(egso *o, int C, const egso_unit *units, int n, uint8_t *valid, int64_t *score, uint8_t *alloc_mask) {
+  if (C < 1 || C > 4 || n < 0 || n > o->nn) return ST_BAD_ARG;
+  uint32_t shape = intern(o, C, units);
+  uint32_t key = node_key(o, shape, C, units);
+  for (int i = 0; i < n; i++) {
+    opt_t *hit = cache_find(&o->nodes[i], key);
+    valid[i] = hit != NULL;
+    score[i] = hit ? hit->score : 0;
+    for (int c = 0; c < 4; c++) {
+      uint8_t m = 0;
+      if (hit && c < C)
+        for (int k = 0; k < hit->n[c]; k++) m |= (uint8_t)(1u << hit->idx[c][k]);
+      alloc_mask[(size_t)i * 4 + c] = m;
+    }
+  }
+  return ST_OK;
+}
 /* AddPod scheduler.go:229-245 */
 int egso_add_pod(egso *o, int node, int C, const egso_unit *units, const int32_t *alloc_off,
                  const int32_t *alloc_idx, uint64_t uid) {

@@ -64,6 +64,7 @@ int egso_forget_pod(egso *o, int node, int C, const egso_unit *units,
 /* TEST SUPPORT: load cached options of one shape (a scheduler that already ran); see egs_oracle.c */
 int egso_cache_load(egso *o, int C, const egso_unit *units, int n, const int32_t *node_ids,
                     const uint8_t *valid, const int64_t *score, const uint8_t *alloc_mask);
+int egso_cache_dump(egso *o, int C, const egso_unit *units, int n, uint8_t *valid, int64_t *score, uint8_t *alloc_mask);
 int egso_known_pod(egso *o, uint64_t uid);
 int egso_released_pod(egso *o, uint64_t uid);
 

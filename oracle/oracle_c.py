@@ -57,6 +57,7 @@ def lib():
         L.egso_add_pod.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64]
         L.egso_forget_pod.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64]
         L.egso_cache_load.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.egso_cache_dump.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
         L.egso_known_pod.argtypes = [C.c_void_p, C.c_uint64]
         L.egso_released_pod.argtypes = [C.c_void_p, C.c_uint64]
         L.egso_schedule_batch.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int] + \
@@ -179,6 +180,16 @@ class OracleC:
         sc = np.ascontiguousarray(score, dtype=np.int64)
         am = np.ascontiguousarray(alloc_mask, dtype=np.uint8)
         return self.L.egso_cache_load(self.h, len(req), _units(req), len(v), None, _ptr(v), _ptr(sc), _ptr(am))
+
+    def cache_dump(self, req, n: Optional[int] = None):
+        """Option cache of request `req` on nodes [0, n): (valid u8[n], score i64[n], alloc_mask u8[n, 4]) --
+        egso_peek of every node in one call, laid out like egso_cache_load's input."""
+        n = self.n_nodes if n is None else n
+        v = np.zeros(max(n, 1), np.uint8); sc = np.zeros(max(n, 1), np.int64); am = np.zeros((max(n, 1), 4), np.uint8)
+        st = self.L.egso_cache_dump(self.h, len(req), _units(req), n, _ptr(v), _ptr(sc), _ptr(am))
+        if st != 0:
+            raise ValueError(f"egso_cache_dump: status {st}")
+        return v[:n], sc[:n], am[:n]
 
     def known_pod(self, uid: int) -> bool:
         return bool(self.L.egso_known_pod(self.h, uid))
